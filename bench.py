@@ -5,6 +5,7 @@
     python bench.py --config cfg3|cfg4 ...                         # the other single-GPU BASELINE.json configurations
     torchrun --nproc-per-node N ... bench.py --gpus N ...          # data parallel, one rank per GPU
     python bench.py --impl reference --steps 3 --warmup 1          # the UNMODIFIED reference train.train on the host cores
+    python bench.py ... --dump-outputs DIR                         # also save the last timed step's results as DIR/*.npy
 
 One "step" = one full training step on one batch of synthetic prior data, driven through the public API
 (`train.build_trainer(...)` -> `Trainer.step`, batches from the prior's `DataLoader`):
@@ -17,6 +18,7 @@ import argparse
 import contextlib
 import json
 import os
+import random
 import subprocess
 import sys
 import threading
@@ -26,6 +28,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 METRIC = "prior-sampled sequences/sec, full training step (prior sample + fwd + bwd + allreduce + clip + Adam)"
@@ -154,6 +157,25 @@ def trainer_args(name, cfg, batch, mods, device, n_steps):
     return prior_mod.DataLoader, crit, enc.Linear, kw
 
 
+DUMP_MAX_ELEMS = 1 << 22      # per dumped array: 16 MB in float32, so the three arrays stay under 64 MB together
+
+
+def dump_sample(t, n=DUMP_MAX_ELEMS):
+    """`t` itself when it has at most `n` elements, else its elements at `n` fixed, seeded positions (flattened)."""
+    if t.numel() <= n:
+        return t
+    idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:n].sort().values
+    return t.flatten()[idx.to(t.device)]
+
+
+def step_outputs(loss, losses, model):
+    """What one Trainer.step hands its caller -- the mean loss, the per-position losses -- and the parameters its optimizer
+    update left in the model, as float32 host tensors (a fixed sample of the concatenated parameters)."""
+    params = torch.cat([p.detach().float().flatten() for p in model.parameters()])
+    return {name: dump_sample(t.detach().float()).cpu()
+            for name, t in (("loss", loss), ("losses", losses), ("params_sample", params))}
+
+
 def randomise_zero_init(model, seed=4321):
     """The reference zero-initialises out_proj / linear2 (transformer.py:43-53): at step 0 dattn, du and dqkv would be
     all-zero tensors, which under an active power cap changes clocks (operand toggling).  The bench measures the
@@ -274,7 +296,9 @@ def run_engine(args):
     B = args.batch or cfg["batch"]
     peaks = load_peaks()
     os.environ["PFN_B200_PRECISION"] = args.precision
-    torch.manual_seed(1234)
+    # every generator a prior draws from (the BNN prior samples its hyperparameters with numpy and random): the same
+    # arguments give the same inputs, so that outputs of two builds can be compared
+    torch.manual_seed(1234); np.random.seed(1234); random.seed(1234)
     mods = {"priors": priors, "bar_distribution": bar_distribution, "encoders": encoders}
     n_total = 2 * (args.warmup + args.steps) + 8
     with contextlib.redirect_stdout(sys.stderr):
@@ -286,11 +310,12 @@ def run_engine(args):
     tr.model.train()
     sep = cfg["sep"]
     batches = iter(tr.dl)                                        # prefetching loader: next batch sampled on a side stream
+    last = {}
 
     def train_step():
         data, targets = next(batches)
-        loss, _ = tr.step(data, targets, sep)
-        return loss
+        last["loss"], last["losses"] = tr.step(data, targets, sep)
+        return last["loss"]
 
     def barrier():
         if world > 1:
@@ -324,6 +349,7 @@ def run_engine(args):
     L.PROFILE_GEMM = None
     launches = L.launch_count()
     clocks = sampler.stop() if rank == 0 else None
+    outputs = step_outputs(last["loss"], last["losses"], tr.model) if args.dump_outputs and rank == 0 else None
     # Roofline pass for the dominant kernel: the same steps, but with the prior sampled on the MAIN stream (prefetch off), so
     # that no other kernel runs inside the CUDA-event brackets of the GEMM launches (in the timed region above the sampler
     # of the next batch shares the SMs with them, which inflates the bracketed durations without changing the step time).
@@ -385,6 +411,10 @@ def run_engine(args):
 
     if rank != 0:
         return
+    if outputs is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for key, t in outputs.items():
+            np.save(os.path.join(args.dump_outputs, key + ".npy"), t.numpy())
     flops = step_flops(cfg["T"], B, cfg["F"], cfg["E"], cfg["nhid"], cfg["L"], cfg["n_out"], sep)
     achieved_step = flops * args.steps / (ms / 1e3) / 1e12
     # dominant kernel: the tcgen05 GEMM (all dense-layer launches of the timed region, CUDA events on the launch stream)
@@ -464,7 +494,12 @@ def main():
     ap.add_argument("--ref-batch", type=int, default=4, help="bounded CPU sample: sequences per CPU step")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-eager-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last one's loss, per-position losses and a fixed sample of the "
+                         "updated parameters to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs saves the CUDA engine's step (--impl b200)")
     # The contract is ONE JSON line on stdout.  Libraries write there too (NCCL prints its version banner on fd 1 when
     # NCCL_DEBUG is set), so fd 1 points at stderr while the run is in progress and the line goes to the saved descriptor.
     global _REAL_STDOUT

@@ -3,7 +3,7 @@
 This is what `bench.py --impl reference` and the `cpu_baseline` leg time on the GPU box's host cores (kind "port":
 /root/reference does not travel to the GPU box, and its priors need gpytorch which is not installed anywhere).
 It follows the reference's own execution path, not the engine's shortcuts:
-  * GP prior draw: dense RBF kernel + torch.linalg.cholesky + matmul (priors/fast_gp.py:48-56 via gpytorch)
+  * GP prior draw: dense RBF kernel + Cholesky with gpytorch's jitter escalation + matmul (priors/fast_gp.py:48-56)
   * dense [T,T] float mask built on the host every step (transformer.py:35-41,65)
   * nn.TransformerEncoder (post-norm, GELU) over all T rows, decoder on all rows then sliced (transformer.py:84-91)
   * FullSupportBarDistribution in plain torch ops (bar_distribution.py:89-108), mean loss, clip 1.0, Adam (train.py:92-97)
@@ -36,11 +36,22 @@ class RefStyleModel(nn.Module):
         return self.decoder(self.transformer_encoder(src, mask))[sep:]
 
 
+def psd_safe_cholesky(K):
+    """torch.linalg.cholesky with the escalation of gpytorch's psd_safe_cholesky, which the reference's GP draw goes
+    through: when a factorisation fails, 1e-6, 1e-5, then 1e-4 is added to the diagonal of the whole batch."""
+    eye = torch.eye(K.shape[-1], dtype=K.dtype)
+    for jitter in (0.0, 1e-6, 1e-5, 1e-4):
+        Lc, info = torch.linalg.cholesky_ex(K + jitter * eye if jitter else K)
+        if not info.any():
+            return Lc
+    raise torch.linalg.LinAlgError("kernel matrix not positive definite even with jitter 1e-4")
+
+
 def sample_fast_gp_cpu(B, T, F, hps):
     x = torch.rand(B, T, F)
     ls = torch.full((B, F), float(hps["lengthscale"]))
     K = O.gp_kernel_ref(x, ls, torch.full((B,), float(hps["outputscale"])), torch.full((B,), float(hps["noise"])))
-    Lc = torch.linalg.cholesky(K)
+    Lc = psd_safe_cholesky(K)
     y = (Lc @ torch.randn(B, T, 1)).squeeze(-1)
     return x.transpose(0, 1).contiguous(), y.transpose(0, 1).contiguous()
 

@@ -11,6 +11,7 @@ import os
 import random
 import sys
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -38,6 +39,41 @@ CONFIG_CASES = {
     "cfg4_b2": dict(T=2000, B=2, F=1, E=512, nhid=1024, L=6, H=4, n_out=100, sep=1000, seed=105, head="bar"),
 }
 N_PROBE = 96   # gradient elements stored per parameter tensor (seeded positions), for per-element comparisons
+
+PE_CLASSES = ("NoPositionalEncoding", "PositionalEncoding", "LearnedPositionalEncoding", "PairedScrambledPositionalEncodings")
+SCHEDULE_CASES = [(0, 10, 0.5), (3, 10, 0.5), (5, 40, 1.5), (10, 10, 0.5)]     # (warmup, total, cosine cycles)
+SEP_SAMPLERS = ("get_weighted_single_eval_pos_sampler", "get_uniform_single_eval_pos_sampler")
+MLP_T, MLP_B, MLP_G, MLP_F = 64, 256, 8, 18      # BNN prior batch: seq_len, datasets, datasets per model, features
+MLP_SEEDS = (1, 2)
+
+
+def mlp_prior_hyperparameters(u):
+    """The shipped BNN-prior configuration (reference tabular.py:47-70 / TabularEvalSimple.ipynb:154-176); `u` is a
+    priors.utils module providing the samplers."""
+    return (lambda: 3, u.scaled_beta_sampler_f(2, 4, 150, 2), torch.nn.Tanh, u.gamma_sampler_f(3.62, .0677),
+            u.gamma_sampler_f(1.87, .0528), lambda: 0.0, True, u.scaled_beta_sampler_f(1, 1.6, 18, 2), None, False, None,
+            None, None, True, True, lambda n: ([], []), 0.0)
+
+
+def mlp_prior_stats(x, y):
+    """Per-dataset statistics of a BNN prior batch: what a different implementation of the same prior must reproduce."""
+    x, y = x.double().cpu(), y.double().cpu()
+    used = (x.abs().sum(0) > 0).sum(-1).double()
+    xc, yc = x - x.mean(0), y - y.mean(0)
+    corr = (xc * yc.unsqueeze(-1)).sum(0) / (xc.norm(dim=0) * yc.norm(dim=0).unsqueeze(-1) + 1e-12)
+    halves_monotone = all(((y[k::2, i].diff() >= 0).all() or (y[k::2, i].diff() <= 0).all()) for i in range(y.shape[1]) for k in (0, 1))
+    return dict(ymean=y.mean(0), used=used, maxcorr=corr.abs().max(-1).values, xscale=x.std(0).sum(-1) / used.clamp(min=1),
+                halves_monotone=halves_monotone)
+
+
+def seed_all(s):
+    np.random.seed(s); random.seed(s); torch.manual_seed(s)
+
+
+def sep_sampler_draws(mod, fn, n):
+    """Three fresh samplers drawn once each, then one sampler drawn 20 times, after random.seed(n)."""
+    random.seed(n)
+    return [getattr(mod, fn)(n)() for _ in range(3)] + [f() for f in [getattr(mod, fn)(n)] for _ in range(20)]
 
 
 def grad_probe_index(numel, seed):
@@ -127,7 +163,7 @@ def main():
         torch.save({
             "case": case,
             "weights_checksum": checksum(model.state_dict()),
-            "logits": logits.detach(), "losses": losses.detach(), "loss": loss.detach(),
+            "logits": logits.detach().clone(), "losses": losses.detach(), "loss": loss.detach(),
             "grad_checksum": {k: (float(g.double().sum()), float(g.double().abs().sum()), float(g.double().norm()))
                               for k, g in grads.items()},
             "grad_samples": {k: g.flatten()[:16].clone() for k, g in grads.items()},
@@ -159,7 +195,8 @@ def main():
         torch.save({
             "case": case,
             "weights_checksum": checksum(model.state_dict()),
-            "logits": logits.detach().to(torch.float32), "losses": losses.detach(), "loss": loss.detach(),
+            # clone: the logits are a view of the whole (T, B, n_out) output, whose storage torch.save would write in full
+            "logits": logits.detach().to(torch.float32).clone(), "losses": losses.detach(), "loss": loss.detach(),
             "grad_checksum": {k: (float(p.grad.double().sum()), float(p.grad.double().abs().sum()), float(p.grad.double().norm()),
                                   float(p.grad.double().abs().max()))
                               for k, p in model.named_parameters()},
@@ -227,7 +264,66 @@ def main():
     torch.save({"cosine": cos, "linear": lin, "weighted_sep": weighted, "uniform_sep": uniform,
                 "openai_lr": ref_utils.get_openai_lr(lr_model), "openai_lr_nparams": sum(p.numel() for p in lr_model.parameters())},
                os.path.join(OUT, "utils.pt"))
+    reference_module_fixtures(_load_ref("positional_encodings"), ref_utils)
+    checkpoint_layout_fixture()
+    mlp_prior_fixture()
     print("golden fixtures written to", OUT)
+
+
+def reference_module_fixtures(ref_pe, ref_utils):
+    """positional_encodings.py (all four classes: initial state, output, RNG consumption) and utils.py (every step of both
+    schedules, the sep samplers, SeqBN) -> ref_modules.pt."""
+    torch.manual_seed(0)
+    x = torch.randn(7, 3, 12)
+    pe = {"x": x}
+    for name in PE_CLASSES:
+        torch.manual_seed(11); m = getattr(ref_pe, name)(12, 20)
+        torch.manual_seed(5); out = m(x).detach()
+        torch.manual_seed(5); m(x); after = torch.rand(4)
+        pe[name] = {"state": m.state_dict(), "out": out, "rand_after": after}
+    schedules = {}
+    for warm, total, cycles in SCHEDULE_CASES:
+        for fn, kw in (("get_cosine_schedule_with_warmup", dict(num_cycles=cycles)), ("get_linear_schedule_with_warmup", {})):
+            opt = torch.optim.SGD([torch.nn.Parameter(torch.zeros(1))], lr=0.7)
+            s = getattr(ref_utils, fn)(opt, warm, total, **kw)
+            cur = []
+            for _ in range(total + 5):
+                cur.append(s.get_last_lr()[0]); opt.step(); s.step()
+            schedules[f"{fn}/{warm}/{total}"] = cur
+    samplers = {f"{fn}/{n}": sep_sampler_draws(ref_utils, fn, n) for n in (1, 2, 37) for fn in SEP_SAMPLERS}
+    torch.manual_seed(0); bn = ref_utils.SeqBN(6)
+    bx = torch.randn(5, 4, 6)
+    seqbn = {"keys": list(bn.state_dict()), "x": bx, "out": bn(bx).detach()}
+    torch.save({"positional_encodings": pe, "schedules": schedules, "sep_samplers": samplers, "seqbn": seqbn},
+               os.path.join(OUT, "ref_modules.pt"))
+
+
+def checkpoint_layout_fixture():
+    """State-dict layout (key order and shapes) of the model checkpoints shipped in the reference's results/ ->
+    checkpoints.pt; the weights themselves are not needed to check that they load."""
+    res = os.path.join(REF, "results")
+    layout = {}
+    for fn in sorted(os.listdir(res)):
+        sd = torch.load(os.path.join(res, fn), map_location="cpu", weights_only=False)[0]
+        layout[fn] = [(k, list(v.shape), str(v.dtype).replace("torch.", "")) for k, v in sd.items()]
+    torch.save(layout, os.path.join(OUT, "checkpoints.pt"))
+
+
+def mlp_prior_fixture():
+    """Statistics of the reference BNN prior (priors/mlp.py through the vendored oracle/_ref tree) on CPU -> mlp_prior.pt."""
+    if ROOT not in sys.path:
+        sys.path.insert(0, ROOT)
+    from oracle import build_ref, ref_runner
+    build_ref.build(verbose=False)
+    mods = ref_runner.load()
+    stats = {}
+    for seed in MLP_SEEDS:
+        seed_all(seed)
+        x, y, _ = mods["priors"].mlp.get_batch(MLP_B, MLP_T, MLP_F, device='cpu',
+                                               hyperparameters=mlp_prior_hyperparameters(mods["priors"].utils),
+                                               batch_size_per_gp_sample=MLP_G)
+        stats[seed] = mlp_prior_stats(x, y)
+    torch.save(stats, os.path.join(OUT, "mlp_prior.pt"))
 
 
 if __name__ == "__main__":

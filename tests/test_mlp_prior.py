@@ -1,46 +1,19 @@
-"""priors.mlp (BNN tabular prior) against the UNMODIFIED reference priors/mlp.py (oracle/_ref, vendored by oracle/build_ref.py):
-same host hyper-sampler stream, same per-dataset distribution.  The vectorised all-models-at-once formulation is checked on
-CPU here (no kernels involved: it is batched torch ops) and on the GPU through the public `get_batch`."""
-import random
+"""priors.mlp (BNN tabular prior) against the UNMODIFIED reference priors/mlp.py (statistics of its batches stored by
+oracle/make_golden.py in golden/mlp_prior.pt): same host hyper-sampler stream, same per-dataset distribution.  The vectorised
+all-models-at-once formulation is checked on CPU here (no kernels involved: it is batched torch ops) and on the GPU through
+the public `get_batch`."""
+import os
 
-import numpy as np
 import pytest
 import torch
 
-from oracle import ref_runner as R
+from oracle.make_golden import MLP_B as B, MLP_F as F, MLP_G as G, MLP_T as T
+from oracle.make_golden import mlp_prior_hyperparameters as _hp, mlp_prior_stats as _stats, seed_all as _seed
 from transformerscandobayesianinference_b200.priors import mlp, utils as su
-
-T, B, G, F = 64, 256, 8, 18
-
-
-def _hp(u):
-    """The shipped BNN-prior configuration (reference tabular.py:47-70 / TabularEvalSimple.ipynb:154-176)."""
-    return (lambda: 3, u.scaled_beta_sampler_f(2, 4, 150, 2), torch.nn.Tanh, u.gamma_sampler_f(3.62, .0677),
-            u.gamma_sampler_f(1.87, .0528), lambda: 0.0, True, u.scaled_beta_sampler_f(1, 1.6, 18, 2), None, False, None,
-            None, None, True, True, lambda n: ([], []), 0.0)
-
-
-def _stats(x, y):
-    x, y = x.double().cpu(), y.double().cpu()
-    used = (x.abs().sum(0) > 0).sum(-1).double()
-    xc, yc = x - x.mean(0), y - y.mean(0)
-    corr = (xc * yc.unsqueeze(-1)).sum(0) / (xc.norm(dim=0) * yc.norm(dim=0).unsqueeze(-1) + 1e-12)
-    halves_monotone = all(((y[k::2, i].diff() >= 0).all() or (y[k::2, i].diff() <= 0).all()) for i in range(y.shape[1]) for k in (0, 1))
-    return dict(ymean=y.mean(0), used=used, maxcorr=corr.abs().max(-1).values, xscale=x.std(0).sum(-1) / used.clamp(min=1),
-                halves_monotone=halves_monotone)
-
-
-def _seed(s):
-    np.random.seed(s); random.seed(s); torch.manual_seed(s)
 
 
 def _reference_batch(seed):
-    if not R.available():
-        pytest.skip("oracle/_ref not built (run oracle/build_ref.py where /root/reference exists)")
-    mods = R.load()
-    _seed(seed)
-    x, y, _ = mods["priors"].mlp.get_batch(B, T, F, device='cpu', hyperparameters=_hp(mods["priors"].utils), batch_size_per_gp_sample=G)
-    return _stats(x, y)
+    return torch.load(os.path.join(os.path.dirname(__file__), "golden", "mlp_prior.pt"))[seed]
 
 
 def _check(ours, ref):
